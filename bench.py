@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — images/sec of the MQ-GLIP-T multi-modal query forward on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl mqdet|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl mqdet|reference] [--dump-outputs DIR]
 
 A step = one forward of ``GeneralizedVLRCNN_New`` (Swin-T -> FPN -> QuerySelector/PreSelect/GCP-BERT -> 6x[BiAttention,
 BERT layer, DyConv] -> dot-product token head -> ATSS post-processing + ml_nms) over one batch of synthetic 800x1333
@@ -15,6 +15,8 @@ random-init weights of the real architecture (no checkpoints offline).
           of the fixed-shape per-image detections per step.
   --impl reference : the CPU oracle (oracle/restate.py — the reference's algorithm restated; its own modules cannot run
           the full forward on CPU, SURVEY.md §8c) on the host cores, one image per step (bounded sample), rank 0 only.
+  --dump-outputs DIR : after the timed steps, rank 0 writes what the last timed step returned as DIR/<name>.npy (float32):
+          inputs and weights come from fixed seeds, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -244,6 +246,8 @@ def run_lvis(args):
         res = step()
         ev[i][1].record()
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"detections": res})  # [chunks, B, max_out + 1, 6]: boxes, score, label; count row last
     clk = clocks.stop() if rank == 0 else None
     ms = sum(a.elapsed_time(b) for a, b in ev) / args.steps
     t = torch.tensor([ms], device=dev)
@@ -334,6 +338,8 @@ def run_gdino(args):
         res = step()
         ev[i][1].record()
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"detections": res})  # [world * B, num_queries + 1, 6]: boxes, score, label; count row last
     launches = ops.launch_count
     if graph is not None:  # launches replayed per step = the launches recorded while capturing
         ops.launch_count = 0
@@ -406,6 +412,23 @@ def finish(world):
     os._exit(0)  # nothing left to finalise; interpreter teardown with NCCL/graph state alive is the other place this can hang
 
 
+DUMP_MAX_ELEMENTS = 1 << 21  # per array (8 MB of float32): larger outputs are written as a fixed, seeded sample of their entries
+
+
+def dump_outputs(out_dir, arrays):
+    """{name: device tensor} -> out_dir/<name>.npy as float32.  An array of more than DUMP_MAX_ELEMENTS entries is written as the
+    entries at DUMP_MAX_ELEMENTS flat positions drawn from a generator seeded with 0 (the same positions for the same shape)."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        x = t.detach().float()
+        if x.numel() > DUMP_MAX_ELEMENTS:
+            idx = torch.randint(x.numel(), (DUMP_MAX_ELEMENTS,), generator=torch.Generator().manual_seed(0))
+            x = x.reshape(-1)[idx.to(x.device)]
+        np.save(os.path.join(out_dir, f"{name}.npy"), x.cpu().numpy())
+
+
 def build_inputs(B, seed):
     import torch
     from tools import synth  # synthetic weights/inputs generator (not the measured path)
@@ -470,7 +493,13 @@ def main():
                     help="coco: BASELINE config 2 (the headline metric); lvis: BASELINE config 3 (MQ-GLIP-L, chunked 1203-class prompt); "
                          "gdino: BASELINE config 4 (MQ-GroundingDINO-T, 2 images / GPU, 13-class prompt)")
     ap.add_argument("--chunks-per-pass", type=int, default=4)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (float32; large arrays as a fixed, seeded sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the CUDA path (--impl mqdet)")
     if args.impl == "reference":
         return run_reference(args)
     if args.config == "lvis":
@@ -565,6 +594,11 @@ def main():
         main_stream.wait_event(e)
     tail[1].record()
     barrier()
+    if args.dump_outputs and rank == 0:
+        # the last timed step: the packed detections InferenceEngine.run turns into BoxLists, and the head outputs they come from
+        last = engine.outs[(args.steps - 1) & 1]
+        dump_outputs(args.dump_outputs, {"detections": last["packed"], "dot_product_logits": last["raw"]["head"]["dot_product_logits"],
+                                         "reg_ctr": last["raw"]["head"]["reg_ctr"], "fused_language": last["raw"]["head"]["hidden"]})
     launches = launches_per_step * args.steps
     ms = (sum(a.elapsed_time(b) for a, b in ev) + tail[0].elapsed_time(tail[1])) / args.steps
     t = torch.tensor([ms], device=dev)

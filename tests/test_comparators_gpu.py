@@ -1,9 +1,9 @@
 """Same-box speed comparators (BASELINE.md §3, SURVEY.md §2.3 / §8d; VERDICT round 1 "missing" item 6) — measurements recorded
 as a GPU test because only tests/ may touch oracle/ and oracle/_ref:
 
-  * the reference's own CUDA kernels, built unmodified for sm_100a (oracle/_ref/mqdet_ref_C.so): ``ml_nms`` and
-    ``modulated_deform_conv_forward`` next to ``mqdet_ml_nms`` / ``mqdet_dcn_cols`` + the tcgen05 GEMM at the bench operating
-    point ("beat the reference kernel compiled for sm_100a on the same box");
+  * the reference's own CUDA kernels, built unmodified for sm_100a (oracle/_ref/mqdet_ref_C.so, timed where it has been built):
+    ``ml_nms`` and ``modulated_deform_conv_forward`` next to ``mqdet_ml_nms`` / ``mqdet_dcn_cols`` + the tcgen05 GEMM at the bench
+    operating point ("beat the reference kernel compiled for sm_100a on the same box");
   * the reference ALGORITHM in eager PyTorch on the same B200 (oracle/restate.py moved to CUDA: the reference modules themselves
     cannot be imported on the GPU box) for one GCP block and one BiAttention fusion layer at the BASELINE config 2 shapes
     ("fused GCP kernel vs reference PyTorch attention"), fp32 and fp16 autocast.
@@ -102,7 +102,7 @@ def test_speed_comparators(dev):
     boxes, scores, labels = _boxes(77, 3600, 80)
     scores = scores + torch.arange(3600) * 1e-7
     b, s, l = boxes.to(dev), scores.to(dev), labels.to(dev)
-    out["ml_nms_3600x80"] = {"reference_kernel_ms": _time(lambda: ref.ml_nms(b, s, l, 0.6)),
+    out["ml_nms_3600x80"] = {"reference_kernel_ms": _time(lambda: ref.ml_nms(b, s, l, 0.6)) if ref else None,
                              "mqdet_ms": _time(lambda: ops.ml_nms_device(b, s, l, 0.6)),
                              "note": "reference = ATen sort + nms kernel + D2H of the mask + host scan (csrc/cuda/ml_nms.cu:79-149); "
                                      "mqdet = device argsort + bitmask + device scan, no D2H"}
@@ -130,7 +130,7 @@ def test_speed_comparators(dev):
 
     y_i, y_c = ours_implicit().float(), ours().float()
     assert (y_i - y_c).abs().max().item() <= 2e-3 * y_c.abs().max().item()
-    out["dcnv2_3x3_B8_100x168_256ch"] = {"reference_kernel_ms": _time(lambda: _ref_dcn(ref, x, off, msk, w, bias, 1)),
+    out["dcnv2_3x3_B8_100x168_256ch"] = {"reference_kernel_ms": _time(lambda: _ref_dcn(ref, x, off, msk, w, bias, 1)) if ref else None,
                                          "mqdet_ms": _time(ours_implicit), "mqdet_cols_gemm_ms": _time(ours),
                                          "note": "reference = fp32 im2col + per-image SGEMM (deform_conv_cuda.cu:496-575); "
                                                  "mqdet = implicit GEMM (mqdet_dcn_conv: sampling fused into the tcgen05 mainloop, "

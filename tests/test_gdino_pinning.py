@@ -1,20 +1,19 @@
 """CPU, build container only: pins the GroundingDINO part of oracle/restate.py (BASELINE config 4, SURVEY.md §8 f1) against the
-reference's own code executed from /root/reference — the whole ``Transformer.forward`` (encoder with fusion + text enhancer +
+reference's own code — the whole ``Transformer.forward`` (encoder with fusion + text enhancer +
 deformable layers, two-stage selection, decoder with iterative box refinement), ``PositionEmbeddingSineHW``, the per-category text
 masks of bertwarper.py, the GroundingDINO Swin-T backbone, the BERT loop under a per-query mask with restarted position ids, and
 ``convert_groundingdino_to_glip_output``.  Also checks the product's host-side helpers (no GPU needed) against the same code.
-Skipped where the reference is absent (GPU box)."""
+The reference's outputs on the seeded inputs are stored under tests/golden/reference/gdino_pinning.pt (recorded where its
+sources are present: see util.reference_outputs)."""
 import ast
 import os
 import types
 import warnings
 
-import pytest
 import torch
 
 from oracle import make_golden, ref_loader, restate, synth
-
-pytestmark = pytest.mark.skipif(not ref_loader.available(), reason="/root/reference not present")
+from util import ref_close, ref_equal, reference_outputs
 
 TKW = dict(d_model=256, nhead=8, dim_feedforward=2048, dropout=0.0, activation="relu", return_intermediate_dec=True, query_dim=4,
            num_feature_levels=4, enc_n_points=4, dec_n_points=4, learnable_tgt_init=True, two_stage_type="standard",
@@ -23,8 +22,11 @@ TKW = dict(d_model=256, nhead=8, dim_feedforward=2048, dropout=0.0, activation="
 
 
 def _close(a, b, tol=2e-5):
-    err = (a - b).abs().max().item()
-    assert err <= tol * b.abs().max().item() + 1e-6, f"{err:.3e}"
+    ref_close(a, b, tol)
+
+
+def _ref(case, compute, full=()):
+    return reference_outputs("gdino_pinning", case, compute, full)
 
 
 def small_case(gen, B=2, Tt=32, used=25, shapes=((12, 16), (6, 8), (3, 4), (2, 2))):
@@ -72,54 +74,68 @@ def test_gdino_transformer_vs_reference():
     sd = synth.gdino_transformer_sd(gen, el, dl, nq=nq)
     srcs, masks, enc_text, tmask, pid, sam = small_case(gen)
     poss = [restate.position_embedding_sine_hw(m) for m in masks]
-    T = ref_transformer(sd, nq, el, dl)
-    td = {"encoded_text": enc_text.clone(), "text_token_mask": tmask, "position_ids": pid, "text_self_attention_masks": sam}
-    with torch.no_grad(), warnings.catch_warnings():
-        warnings.simplefilter("ignore")
-        hs, refs, hs_enc, ref_enc, init = T(srcs, masks, None, poss, None, None, td)
+
+    def compute():
+        T = ref_transformer(sd, nq, el, dl)
+        td = {"encoded_text": enc_text.clone(), "text_token_mask": tmask, "position_ids": pid, "text_self_attention_masks": sam}
+        with torch.no_grad(), warnings.catch_warnings():
+            warnings.simplefilter("ignore")
+            hs, refs, hs_enc, ref_enc, init = T(srcs, masks, None, poss, None, None, td)
+        return {"hs": hs, "refs": refs, "text": td["encoded_text"], "padding_effect": (hs[-1][0] - hs[-1][1]).abs().max().item(),
+                "fusion_effect": (td["encoded_text"] - enc_text).abs().max().item()}
+    ref = _ref("transformer", compute)
+    hs, refs = ref["hs"], ref["refs"]
     out = restate.gdino_transformer(srcs, masks, poss, enc_text, tmask, pid, sam, sd, num_queries=nq, enc_layers=el, dec_layers=dl)
     assert len(hs) == dl and len(refs) == dl + 1
     for a, b in zip(hs, out["hs"]):
         _close(b, a)
     for a, b in zip(refs, out["references"]):
         _close(b, a)
-    _close(out["memory_text"], td["encoded_text"])
+    _close(out["memory_text"], ref["text"])
     # the padded image differs from the un-padded one, the text stream is changed by the fusion layers
-    assert (hs[-1][0] - hs[-1][1]).abs().max() > 1e-2 and (td["encoded_text"] - enc_text).abs().max() > 1e-2
+    assert ref["padding_effect"] > 1e-2 and ref["fusion_effect"] > 1e-2
+    assert (out["hs"][-1][0] - out["hs"][-1][1]).abs().max() > 1e-2 and (out["memory_text"] - enc_text).abs().max() > 1e-2
 
 
 def test_position_embedding_vs_reference():
     import importlib
-    p = ref_loader.gdino_package()
-    pe = importlib.import_module("ref_gdino_pkg.backbone.position_encoding")
-    mod = pe.PositionEmbeddingSineHW(128, temperatureH=20, temperatureW=20, normalize=True)
-    misc = importlib.import_module("groundingdino_new.util.misc")
     m = torch.zeros(2, 13, 17, dtype=torch.bool)
     m[1, 9:, :] = True
     m[1, :, 12:] = True
-    ref = mod(misc.NestedTensor(torch.zeros(2, 256, 13, 17), m))
+
+    def compute():
+        ref_loader.gdino_package()
+        pe = importlib.import_module("ref_gdino_pkg.backbone.position_encoding")
+        mod = pe.PositionEmbeddingSineHW(128, temperatureH=20, temperatureW=20, normalize=True)
+        misc = importlib.import_module("groundingdino_new.util.misc")
+        return {"pos": mod(misc.NestedTensor(torch.zeros(2, 256, 13, 17), m))}
+    ref = _ref("position_embedding", compute)["pos"]
     got = restate.position_embedding_sine_hw(m)
-    assert torch.equal(got, ref)
+    assert ref_equal(got, ref)
     from mqdet_b200.modeling.groundingdino.groundingdino import PositionEmbeddingSineHW
-    assert torch.equal(PositionEmbeddingSineHW(128, 20, 20)(m), ref)
+    assert ref_equal(PositionEmbeddingSineHW(128, 20, 20)(m), ref)
 
 
 def test_text_masks_vs_reference():
     import importlib
-    ref_loader.gdino_package()
-    bw = importlib.import_module("ref_gdino_pkg.bertwarper")
     gen = synth.Gen(72)
     ids, am, pmap = synth.prompt(13, 2, 64, gen)
     ids_b, _, _ = synth.prompt(7, 3, 64, gen)
     ids2 = torch.cat([ids, ids_b], 0)  # second row: other category lengths (the reference carries previous_col across rows)
     special = [101, 102, 1012, 1029]
-    rm, rp, rc = bw.generate_masks_with_special_tokens_and_transfer_map({"input_ids": ids2}, special, None)
+
+    def compute():
+        ref_loader.gdino_package()
+        bw = importlib.import_module("ref_gdino_pkg.bertwarper")
+        return dict(zip(("mask", "pos", "cate"), bw.generate_masks_with_special_tokens_and_transfer_map({"input_ids": ids2}, special, None)))
+    ref = _ref("text_masks", compute, full=("mask", "pos", "cate"))
+    rm, rp, rc = ref["mask"], ref["pos"], ref["cate"]
     gm, gp = restate.gdino_text_masks(ids2, special)
     assert torch.equal(gm, rm) and torch.equal(gp, rp)
     from mqdet_b200.modeling.groundingdino.bertwarper import generate_masks_with_special_tokens_and_transfer_map as mine
     pm, pp, pc = mine({"input_ids": ids2}, special)
     assert torch.equal(pm, rm) and torch.equal(pp, rp)
-    assert all(torch.equal(a, b) for a, b in zip(pc, rc))
+    assert len(pc) == len(rc) and all(torch.equal(a, b) for a, b in zip(pc, rc))
     # every category of the synthetic prompt is a block: its tokens see each other and the trailing '.', nothing else
     toks = pmap[1]
     assert rm[0, toks[0], toks[-1]] and not rm[0, toks[0], pmap[2][0]]
@@ -127,22 +143,25 @@ def test_text_masks_vs_reference():
 
 def test_gdino_swin_vs_reference():
     import importlib
-    ref_loader.gdino_package()
-    with warnings.catch_warnings():
-        warnings.simplefilter("ignore")
-        st = importlib.import_module("ref_gdino_pkg.backbone.swin_transformer")
-        model = st.build_swin_transformer("swin_T_224_1k", 224, out_indices=(1, 2, 3), dilation=False, use_checkpoint=False)
-        model.eval()  # the reference overrides train() without returning self
     gen = synth.Gen(73)
     sd = synth.swin_sd(gen)
-    own = model.state_dict()
-    load = {k: sd[k] for k in own if k in sd}
-    missing = [k for k in own if k not in sd and not k.endswith(("relative_position_index", "attn_mask"))]
-    assert not missing, missing[:5]
-    model.load_state_dict(load, strict=False)
     img = synth.rgb_images(gen, 2, 75, 110)
-    with torch.no_grad():
-        ref = model.forward_raw(img)
+
+    def compute():
+        ref_loader.gdino_package()
+        with warnings.catch_warnings():
+            warnings.simplefilter("ignore")
+            st = importlib.import_module("ref_gdino_pkg.backbone.swin_transformer")
+            model = st.build_swin_transformer("swin_T_224_1k", 224, out_indices=(1, 2, 3), dilation=False, use_checkpoint=False)
+            model.eval()  # the reference overrides train() without returning self
+        own = model.state_dict()
+        load = {k: sd[k] for k in own if k in sd}
+        missing = [k for k in own if k not in sd and not k.endswith(("relative_position_index", "attn_mask"))]
+        assert not missing, missing[:5]
+        model.load_state_dict(load, strict=False)
+        with torch.no_grad():
+            return {"outs": model.forward_raw(img)}
+    ref = _ref("swin", compute)["outs"]
     got = restate.swin_transformer(img, sd)[1:]
     assert len(ref) == 3
     for a, b in zip(ref, got):
@@ -154,44 +173,48 @@ def test_bert_loop_with_category_masks_vs_reference():
     get_extended_attention_mask builds from a 3-D mask (bertwarper.py:141-143), on the reference's own classes."""
     import torch.nn as nn
     from transformers import BertConfig
-    m, rb = ref_loader.modeling_bert_new(), ref_loader.rpn_modeling_bert()
     config = BertConfig(num_hidden_layers=2)
     gen = synth.Gen(74)
     sd = synth.qvbert_sd(gen, layers=2, start_qv=1)
-    emb = m.QVBertEmbeddings(config, make_golden.ref_cfg()).eval()
-    emb.load_state_dict({k: sd["embeddings." + k] for k in emb.state_dict() if "embeddings." + k in sd}, strict=False)
-    if not hasattr(emb, "position_embedding_type"):  # transformers-4 BertEmbeddings attribute (BertConfig default)
-        emb.position_embedding_type = "absolute"
     ids, am, pmap = synth.prompt(10, 2, 64, gen)
     self_mask, pid = restate.gdino_text_masks(ids)
-    with torch.no_grad():
-        ref_e = emb(input_ids=ids, position_ids=pid, token_type_ids=torch.zeros_like(ids))
-    _close(restate.bert_embeddings(ids, sd, position_ids=pid), ref_e)
-
-    class Layer(nn.Module):
-        def __init__(self):
-            super().__init__()
-            self.attention = rb.BertAttention(config, False, False)
-            self.intermediate = rb.BertIntermediate(config)
-            self.output = rb.BertOutput(config)
-
-        def forward(self, h, attention_mask=None, head_mask=None, enc_h=None, enc_mask=None, past=None, output_attentions=False):
-            a = self.attention(h, attention_mask, None, output_attentions=False, past_key_value=None)[0]
-            return (self.output(self.intermediate(a), a),)
-
-    enc = m.QVBertEncoder(config, dim=768, cfg=make_golden.ref_cfg(), start_qv_layer_index=1).eval()
-    enc.gradient_checkpointing = False
-    enc.layer = nn.ModuleList([Layer() for _ in range(2)]).eval()
-    enc.load_state_dict({k: sd["encoder." + k] for k in enc.state_dict()}, strict=True)
     ext = (1.0 - self_mask[:, None].float()) * -10000.0
-    with torch.no_grad():
-        ref = enc(ref_e, attention_mask=ext).last_hidden_state
-    got = ref_e
+
+    def compute():
+        m, rb = ref_loader.modeling_bert_new(), ref_loader.rpn_modeling_bert()
+        emb = m.QVBertEmbeddings(config, make_golden.ref_cfg()).eval()
+        emb.load_state_dict({k: sd["embeddings." + k] for k in emb.state_dict() if "embeddings." + k in sd}, strict=False)
+        if not hasattr(emb, "position_embedding_type"):  # transformers-4 BertEmbeddings attribute (BertConfig default)
+            emb.position_embedding_type = "absolute"
+        with torch.no_grad():
+            ref_e = emb(input_ids=ids, position_ids=pid, token_type_ids=torch.zeros_like(ids))
+
+        class Layer(nn.Module):
+            def __init__(self):
+                super().__init__()
+                self.attention = rb.BertAttention(config, False, False)
+                self.intermediate = rb.BertIntermediate(config)
+                self.output = rb.BertOutput(config)
+
+            def forward(self, h, attention_mask=None, head_mask=None, enc_h=None, enc_mask=None, past=None, output_attentions=False):
+                a = self.attention(h, attention_mask, None, output_attentions=False, past_key_value=None)[0]
+                return (self.output(self.intermediate(a), a),)
+
+        enc = m.QVBertEncoder(config, dim=768, cfg=make_golden.ref_cfg(), start_qv_layer_index=1).eval()
+        enc.gradient_checkpointing = False
+        enc.layer = nn.ModuleList([Layer() for _ in range(2)]).eval()
+        enc.load_state_dict({k: sd["encoder." + k] for k in enc.state_dict()}, strict=True)
+        with torch.no_grad():
+            return {"embeddings": ref_e, "hidden": enc(ref_e, attention_mask=ext).last_hidden_state}
+    r = _ref("bert_loop_with_category_masks", compute)
+    emb = restate.bert_embeddings(ids, sd, position_ids=pid)
+    _close(emb, r["embeddings"])
+    ref, got = r["hidden"], emb
     for i in range(2):
         got = restate.bert_layer(got, ext, sd, f"encoder.layer.{i}.", 12)
     _close(got, ref)
-    full = restate.bert_layer(ref_e, None, sd, "encoder.layer.0.", 12)
-    assert (full - restate.bert_layer(ref_e, ext, sd, "encoder.layer.0.", 12)).abs().max() > 1e-3  # the block mask matters
+    full = restate.bert_layer(emb, None, sd, "encoder.layer.0.", 12)
+    assert (full - restate.bert_layer(emb, ext, sd, "encoder.layer.0.", 12)).abs().max() > 1e-3  # the block mask matters
 
 
 def _ref_convert_fn():
@@ -216,7 +239,6 @@ def _ref_convert_fn():
 
 
 def test_gdino_detections_vs_reference():
-    fn = _ref_convert_fn()
     gen = synth.Gen(75)
     B, nq, T, C = 2, 60, 256, 80
     _, am, pmap = synth.prompt(13, 2, T, gen)
@@ -228,10 +250,15 @@ def test_gdino_detections_vs_reference():
     sizes = [(480, 640), (400, 600)]
     me = types.SimpleNamespace(cfg=types.SimpleNamespace(MODEL=types.SimpleNamespace(DYHEAD=types.SimpleNamespace(NUM_CLASSES=C + 1))),
                                box_threshold=0.05)
-    ref = fn(me, {"pred_logits": logits.sigmoid(), "pred_boxes": boxes}, pmap, sizes)
+
+    def compute():
+        ref = _ref_convert_fn()(me, {"pred_logits": logits.sigmoid(), "pred_boxes": boxes}, pmap, sizes)
+        return {"labels": [r.get_field("labels") for r in ref], "scores": [r.get_field("scores") for r in ref], "bbox": [r.bbox for r in ref]}
+    ref = _ref("detections", compute, full=("labels", "scores", "bbox"))
     got = restate.gdino_detections(logits, boxes, pmap, C, sizes, 0.05)
-    for r, (gb, gs, gl) in zip(ref, got):
-        assert len(r) == gb.shape[0] and len(r) > 5
-        assert torch.equal(r.get_field("labels"), gl)
-        _close(gs, r.get_field("scores"), 1e-6)
-        _close(gb, r.bbox, 1e-6)
+    assert len(got) == len(ref["labels"])
+    for rl_, rs, rb, (gb, gs, gl) in zip(ref["labels"], ref["scores"], ref["bbox"], got):
+        assert len(rl_) == gb.shape[0] and len(rl_) > 5
+        assert torch.equal(rl_, gl)
+        _close(gs, rs, 1e-6)
+        _close(gb, rb, 1e-6)

@@ -12,6 +12,7 @@ import pytest
 import torch
 
 from oracle import ref_loader
+from util import reference_outputs
 
 WORDS = ["[PAD]", "[UNK]", "[CLS]", "[SEP]", "[MASK]", ".", "person", "traffic", "light", "fire", "hydrant", "bicycle", "##s", "cat", "dog",
          "tv", "hot", "wine", "glass", "##es", "teddy", "bear", "hair", "drier", "cell", "phone", "potted", "plant", "stop", "sign", "a", "of",
@@ -55,24 +56,28 @@ class _Dataset:
         return dict(NAMES)
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="/root/reference not present")
 @pytest.mark.parametrize("chunk", [-1, 4])
 def test_prompts_vs_reference(tokenizer, chunk):
+    """The reference's outputs are stored under tests/golden/reference/prompts.pt (see util.reference_outputs)."""
     from mqdet_b200.engine import prompts
     tok, tok_dir = tokenizer
-    ref = _reference_functions()
     cfg = _cfg(tok_dir, chunk)
-    rq, rm = ref["create_queries_and_maps_from_dataset"](_Dataset(), cfg, disable_print=True)
-    q, m = prompts.create_queries_and_maps_from_dataset(_Dataset(), cfg, tokenizer=tok)
-    assert q == rq and len(q) == (1 if chunk == -1 else 4)
-    assert [dict(x) for x in m] == [dict(x) for x in rm]
-    assert "stop sign" in q[0] + "".join(q[1:]) and "sports ball" in "".join(q) and "(round)" not in "".join(q)   # clean_name
-    assert prompts.clean_name("sports ball(round)") == ref["clean_name"]("sports ball(round)")
     pm = torch.zeros(3, 16)
     pm[0, 1:3] = 0.5
     pm[2, 7] = 1.0
-    assert prompts.create_positive_map_label_to_token_from_positive_map(pm, plus=1) == \
-        ref["create_positive_map_label_to_token_from_positive_map"](pm, plus=1)
+
+    def compute():
+        ref = _reference_functions()
+        rq, rm = ref["create_queries_and_maps_from_dataset"](_Dataset(), cfg, disable_print=True)
+        return {"queries": rq, "maps": [dict(x) for x in rm], "clean_name": ref["clean_name"]("sports ball(round)"),
+                "label_to_token": dict(ref["create_positive_map_label_to_token_from_positive_map"](pm, plus=1))}
+    ref = reference_outputs("prompts", f"chunk_{chunk}", compute)
+    q, m = prompts.create_queries_and_maps_from_dataset(_Dataset(), cfg, tokenizer=tok)
+    assert q == ref["queries"] and len(q) == (1 if chunk == -1 else 4)
+    assert [dict(x) for x in m] == ref["maps"]
+    assert "stop sign" in q[0] + "".join(q[1:]) and "sports ball" in "".join(q) and "(round)" not in "".join(q)   # clean_name
+    assert prompts.clean_name("sports ball(round)") == ref["clean_name"]
+    assert prompts.create_positive_map_label_to_token_from_positive_map(pm, plus=1) == ref["label_to_token"]
 
 
 def test_prompts_into_token_ids(tokenizer):

@@ -296,7 +296,7 @@ def test_ml_nms_score_ties_equal_reference_kernel(dev):
     from test_nms_gpu import _boxes
     from test_ref_kernels_gpu import _ref
     from mqdet_b200 import ops
-    ref = _ref()
+    from util import reference_outputs
     n, nlabels = 3000, 40
     boxes, _, _ = _boxes(4242, n, nlabels)
     g = torch.Generator().manual_seed(5)
@@ -306,7 +306,9 @@ def test_ml_nms_score_ties_equal_reference_kernel(dev):
     labels = torch.cat([torch.randint(1, nlabels // 2 + 1, (m,), generator=g),
                         torch.randint(nlabels // 2 + 1, nlabels + 1, (m,), generator=g)]).float()   # ... on different labels
     boxes = boxes[: 2 * m]
-    want = ref.ml_nms(boxes.to(dev), scores.to(dev), labels.to(dev), 0.6).cpu()
+    # the reference kernel's kept set, stored under tests/golden/reference/ref_kernels.pt
+    want = reference_outputs("ref_kernels", "ml_nms_score_ties",
+                             lambda: {"keep": _ref().ml_nms(boxes.to(dev), scores.to(dev), labels.to(dev), 0.6)}, full=("keep",))["keep"]
     got = ops.ml_nms(boxes.to(dev), scores.to(dev), labels.to(dev), 0.6).cpu()
     assert torch.equal(got, want)
 

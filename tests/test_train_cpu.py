@@ -1,39 +1,38 @@
-"""CPU: pins the training-side oracle pieces against the reference's own code (build container only) and checks the host-side
-parameter-group rules of mqdet_b200.solver.build against solver/build.py."""
+"""CPU: pins the training-side oracle pieces against the reference's own code, through its outputs on seeded inputs stored under
+tests/golden/reference/train.pt (recorded where the reference's sources are present: see util.reference_outputs), and checks
+the host-side parameter-group rules of mqdet_b200.solver.build against solver/build.py."""
 import types
 
-import pytest
 import torch
 
 from oracle import ref_loader, restate
+from util import ref_close, reference_outputs
 
-needs_ref = pytest.mark.skipif(not ref_loader.available(), reason="/root/reference not present")
 
-
-@needs_ref
 def test_token_focal_loss_vs_reference():
     import sys
-    ref_loader._install_shims()
-    sys.modules["maskrcnn_benchmark"]._C = types.SimpleNamespace()   # the CUDA-only sigmoid focal loss op is not on this path
-    m = ref_loader._load_file("ref_sigmoid_focal_loss", "maskrcnn_benchmark/layers/sigmoid_focal_loss.py")
     g = torch.Generator().manual_seed(4)
     logits = torch.randn(2, 300, 256, generator=g) * 3 - 2
     targets = (torch.rand(2, 300, 256, generator=g) > 0.95).float()
     tm = torch.ones(2, 256)
     tm[0, 200:] = 0
     tm[1, 120:] = 0
-    mod = m.TokenSigmoidFocalLoss(0.25, 2.0)
-    for mask in (tm, None):
-        ref = mod(logits, targets, text_masks=mask, version="binary")
+
+    def compute():
+        ref_loader._install_shims()
+        sys.modules["maskrcnn_benchmark"]._C = types.SimpleNamespace()   # the CUDA-only sigmoid focal loss op is not on this path
+        m = ref_loader._load_file("ref_sigmoid_focal_loss", "maskrcnn_benchmark/layers/sigmoid_focal_loss.py")
+        mod = m.TokenSigmoidFocalLoss(0.25, 2.0)
+        return {"loss": [mod(logits, targets, text_masks=mask, version="binary").item() for mask in (tm, None)]}
+    ref = reference_outputs("train", "token_focal_loss", compute)["loss"]
+    for mask, want in zip((tm, None), ref):
         got = restate.token_focal_loss(logits, targets, 0.25, 2.0, mask)
-        assert abs(ref.item() - got.item()) <= 1e-6 * abs(ref.item())
+        assert abs(want - got.item()) <= 1e-6 * abs(want)
 
 
-@needs_ref
 def test_gcp_block_autograd_oracle_vs_reference():
     """The backward oracle = autograd over restate.gcp_block: its gradients equal autograd over the reference's own block."""
     from oracle import make_golden, synth
-    m = ref_loader.modeling_bert_new()
     gen = synth.Gen(6)
     sd = synth.gcp_block_sd(gen)
     B, T = 2, 64
@@ -42,21 +41,23 @@ def test_gcp_block_autograd_oracle_vs_reference():
     mask = mk.expand(B, -1, -1).clone()
     mask[0, 3] = 0
     vision, x, dy = gen.randn(B, mask.shape[1], 768), gen.randn(B, T, 768), gen.randn(B, T, 768)
-    blk = m.GatedCrossAttentionBlock(dim=768, cfg=make_golden.ref_cfg())
-    blk.load_state_dict(sd, strict=True)
-    xr, vr = x.clone().requires_grad_(True), vision.clone().requires_grad_(True)
-    blk(xr, vr, mask).backward(dy)
+
+    def compute():
+        blk = ref_loader.modeling_bert_new().GatedCrossAttentionBlock(dim=768, cfg=make_golden.ref_cfg())
+        blk.load_state_dict(sd, strict=True)
+        xr, vr = x.clone().requires_grad_(True), vision.clone().requires_grad_(True)
+        blk(xr, vr, mask).backward(dy)
+        return {"x": xr.grad, "vision": vr.grad, "params": {k: q.grad for k, q in blk.named_parameters()}}
+    ref = reference_outputs("train", "gcp_block_autograd", compute)
     p = {k: v.clone().requires_grad_(True) for k, v in sd.items()}
     x2, v2 = x.clone().requires_grad_(True), vision.clone().requires_grad_(True)
     restate.gcp_block(x2, v2, mask, p, "").backward(dy)
 
-    def close(a, b):
-        assert (a - b).abs().max().item() <= 2e-5 * b.abs().max().item() + 1e-7
-
-    close(x2.grad, xr.grad)
-    close(v2.grad, vr.grad)
-    for k, q in blk.named_parameters():
-        close(p[k].grad.view(q.grad.shape), q.grad)
+    ref_close(x2.grad, ref["x"], 2e-5, "x")
+    ref_close(v2.grad, ref["vision"], 2e-5, "vision")
+    assert sorted(ref["params"]) == sorted(k for k in p if p[k].grad is not None)
+    for k, q in ref["params"].items():
+        ref_close(p[k].grad.view(q["sampled"] if isinstance(q, dict) else q.shape), q, 2e-5, k)
 
 
 def test_param_group_rules():

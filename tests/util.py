@@ -1,4 +1,5 @@
 """Shared helpers for the parity tests."""
+import math
 import os
 import sys
 import types
@@ -51,6 +52,91 @@ def assert_close(out, ref, tol=FP16_TOL, what="", defer=None):
         return err
     assert err <= bound, f"{what}: max|err| {err:.3e} > {bound:.3e} (max|ref| {ref.abs().max().item():.3e})"
     return err
+
+
+# ---- outputs of the reference's own code, stored under tests/golden/reference/ ------------------------------------------
+# The pinning tests compare against what the reference's modules / kernels computed on seeded inputs.  Those runs need the
+# reference sources (and, for its CUDA kernels, a GPU), so their outputs are stored: tensors of at most REF_FULL elements
+# whole, larger ones as REF_SAMPLE entries at fixed positions plus max|x| and mean|x| of the whole tensor.
+REFERENCE_DIR = os.path.join(ROOT, "tests", "golden", "reference")
+REF_FULL, REF_SAMPLE = 1024, 256
+
+
+def _sample_positions(numel):
+    """Fixed positions spread over a flat tensor: a stride coprime with ``numel`` visits distinct elements."""
+    stride = 2654435761 % numel or 1
+    while math.gcd(stride, numel) != 1:
+        stride += 1
+    return torch.tensor([(i * stride + 7) % numel for i in range(min(REF_SAMPLE, numel))], dtype=torch.long)
+
+
+def _condense(x, full, keep=False):
+    if isinstance(x, torch.Tensor):
+        x = x.detach().cpu().contiguous()
+        if keep or x.numel() <= REF_FULL:
+            return x.clone()
+        fin = x[torch.isfinite(x)].abs().double() if x.is_floating_point() else x.abs().double()
+        return {"sampled": list(x.shape), "val": x.reshape(-1)[_sample_positions(x.numel())].clone(),
+                "absmax": fin.max().item() if fin.numel() else 0.0, "absmean": fin.mean().item() if fin.numel() else 0.0}
+    if isinstance(x, (list, tuple)):
+        return [_condense(v, full, keep) for v in x]
+    if isinstance(x, dict):
+        return {k: _condense(v, full, keep or k in full) for k, v in x.items()}
+    return x
+
+
+def reference_outputs(fixture, case, compute, full=()):
+    """The stored outputs of the reference for ``case`` (tests/golden/reference/<fixture>.pt).  ``compute`` runs the reference's
+    own code and returns a dict of tensors, lists of tensors and plain values; it runs only when MQDET_RECORD_REFERENCE names a
+    directory, which then receives the condensed result (keys listed in ``full`` are kept whole).  Record with
+    ``MQDET_RECORD_REFERENCE=tests/golden/reference python -m pytest <the test>`` where the reference can run."""
+    out_dir = os.environ.get("MQDET_RECORD_REFERENCE")
+    if not out_dir:
+        return torch.load(os.path.join(REFERENCE_DIR, f"{fixture}.pt"))[case]
+    fx = _condense(compute(), set(full))
+    path = os.path.join(out_dir, f"{fixture}.pt")
+    os.makedirs(out_dir, exist_ok=True)
+    stored = torch.load(path) if os.path.exists(path) else {}
+    stored[case] = fx
+    torch.save(stored, path)
+    return fx
+
+
+def ref_pair(got, ref):
+    """(got, ref) over the entries of the stored reference output ``ref`` (all of them when it was stored whole)."""
+    got = got.detach().cpu()
+    if isinstance(ref, dict):
+        assert list(got.shape) == ref["sampled"], f"shape {tuple(got.shape)} vs {tuple(ref['sampled'])}"
+        return got.reshape(-1)[_sample_positions(got.numel())], ref["val"]
+    assert got.shape == ref.shape, f"shape {tuple(got.shape)} vs {tuple(ref.shape)}"
+    return got, ref
+
+
+def ref_absmax(ref):
+    if isinstance(ref, dict):
+        return ref["absmax"]
+    fin = ref[torch.isfinite(ref)] if ref.is_floating_point() else ref
+    return fin.abs().max().item() if fin.numel() else 0.0
+
+
+def ref_close(got, ref, tol, what="", atol=1e-6):
+    """max|got - ref| <= tol * max|finite ref| + atol over the stored entries (and the same bound on the mean of |x| when
+    sampled); non-finite entries of ref must be matched exactly."""
+    g, r = ref_pair(got, ref)
+    fin = torch.isfinite(r)
+    assert torch.equal(g[~fin], r[~fin]), f"{what}: non-finite entries differ"
+    bound = tol * ref_absmax(ref) + atol
+    err = (g[fin].double() - r[fin].double()).abs().max().item() if fin.any() else 0.0
+    assert err <= bound, f"{what}: {err:.3e} > {bound:.3e}"
+    if isinstance(ref, dict):
+        am = got.detach().cpu().double()
+        am = am[torch.isfinite(am)].abs().mean().item()
+        assert abs(am - ref["absmean"]) <= bound, f"{what}: mean|x| {am:.6e} vs {ref['absmean']:.6e}"
+
+
+def ref_equal(got, ref):
+    g, r = ref_pair(got, ref)
+    return torch.equal(g, r)
 
 
 def vq_cfg(**over):
